@@ -29,6 +29,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -226,16 +228,18 @@ def run_b200(args):
         g = torch.Generator(device=device).manual_seed(99 + M)
         return {K: (torch.randn(M, K, generator=g, device=device) * scale).to(dtype) for K in (cfg["hidden"], cfg["inter"])}
 
-    def abi_graph(M, kind):
-        """CUDA graph of one step: 160 launches through the C ABI on the capture stream."""
+    def abi_graph(M, kind, per_layer=False):
+        """CUDA graph of one step: 160 launches through the C ABI on the capture stream.  Outputs: one buffer per
+        layer with `per_layer`, else one per output width (each layer overwrites the previous one's)."""
         xs = make_inputs(M)
         ys = {N: torch.empty(M, N, dtype=dtype, device=device) for N in {m["N"] for m in model}}
+        outs = [torch.empty(M, m["N"], dtype=dtype, device=device) for m in model] if per_layer else [ys[m["N"]] for m in model]
         fn = lib.b200awq_w4a16_gemv if kind == "gemv" else lib.b200awq_w4a16_gemm
 
         def launch_all():
             st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            for m in model:
-                a = (p(xs[m["K"]]), p(m["qw"]), p(m["sc"]), p(m["sz"]), p(ys[m["N"]]), M, m["N"], m["K"], G, 0)
+            for m, y in zip(model, outs):
+                a = (p(xs[m["K"]]), p(m["qw"]), p(m["sc"]), p(m["sz"]), p(y), M, m["N"], m["K"], G, 0)
                 rc = fn(*a, st) if kind == "gemv" else fn(*a, None, 0, st)
                 if rc != 0:
                     raise RuntimeError(lib.b200awq_strerror(rc).decode())
@@ -246,7 +250,7 @@ def run_b200(args):
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
             launch_all()
-        return g, (xs, ys)
+        return g, (xs, outs)
 
     def plugin_graph(M, kind):
         """CUDA graph of one e2e step: H2D of the activations (pinned), 160 plugin calls, D2H of the result."""
@@ -277,8 +281,8 @@ def run_b200(args):
 
     def eager_e2e(M, steps):
         """The SAME end-to-end step without a CUDA graph: every layer is one eager call of the reference-facing module
-        (the reference's own, unmodified WQLinear.forward when baseline/_ref is staged, else this repo's mirror), as
-        tinychat / awq.entry make them; pinned H2D of the activations and D2H of the result every step."""
+        (this repo's mirror of WQLinear.forward), as tinychat / awq.entry make them; pinned H2D of the activations and
+        D2H of the result every step."""
         mods, kind = reference_wqlinears(torch, model, device, dtype)
         hx = {K: v.cpu().pin_memory() for K, v in make_inputs(M).items()}
         dx = {K: torch.empty_like(v, device=device).view(1, M, K) for K, v in hx.items()}
@@ -293,7 +297,7 @@ def run_b200(args):
             hy.copy_(y, non_blocking=True)
             torch.cuda.current_stream().synchronize()
             _ = float(hy[0, 0, 0])
-        ms, w = timed_steps(torch, dist, device, step, steps, 5)
+        ms, w = timed_steps(torch, dist, device, step, steps, args.warmup)
         # host cost of one call when the GPU is not the bottleneck: issue the calls of one step and stop the clock before
         # waiting for the device
         torch.cuda.synchronize()
@@ -331,8 +335,8 @@ def run_b200(args):
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
                     launch_all()
-                ms, _ = timed_steps(torch, None, device, g.replay, 20, 3)
-                us = ms * 1e3 / 20 / len(layers)
+                ms, _ = timed_steps(torch, None, device, g.replay, args.steps, args.warmup)
+                us = ms * 1e3 / args.steps / len(layers)
                 row["%dx%d" % (N, K)] = {"us": round(us, 3), "frac": round(alg_bytes(M, N, K) / us / 1e3 / peaks["hbm"], 4),
                                          "calls": len(layers)}
             tot_us = sum(v["us"] * v["calls"] for v in row.values())
@@ -341,11 +345,20 @@ def run_b200(args):
             out[str(M)] = row
         return out
 
+    # outputs of the last timed step of each leg (--dump-outputs); prefill outputs at fixed seeded rows
+    dump = {}
+    rows_p = torch.from_numpy(np.sort(np.random.default_rng(0).choice(2048, 64, replace=False)))
+
+    def keep(name, t):
+        dump[name] = t.float().cpu().numpy()
+
     sampler.start()
     # ---------------- decode: device-resident
-    g_dec, keep1 = abi_graph(1, "gemv")
+    g_dec, keep1 = abi_graph(1, "gemv", per_layer=True)
     ms_dec, w = timed_steps(torch, dist, device, g_dec.replay, args.steps, args.warmup)
     windows.append(w)
+    for name, _, _ in layer_projs(cfg):
+        keep("decode_" + name, torch.cat([y for m, y in zip(model, keep1[1]) if m["name"] == name]))
     # ---------------- decode: end to end through the plugin with host buffers
     g_e2e, hy, h2d, d2h = plugin_graph(1, "gemv")
 
@@ -355,22 +368,28 @@ def run_b200(args):
         _ = float(hy[0, 0])            # the host reads the step's result
     ms_e2e, w = timed_steps(torch, dist, device, e2e_step, args.steps, args.warmup)
     windows.append(w)
+    keep("decode_e2e_y", hy)
     # ---------------- prefill (secondary object)
     Mp = 2048
-    ksteps_p = max(3, min(args.steps, args.prefill_steps))
+    ksteps_p = args.steps if args.prefill_steps is None else args.prefill_steps
     g_pre, keep2 = abi_graph(Mp, "gemm")
-    ms_pre, w = timed_steps(torch, dist, device, g_pre.replay, ksteps_p, 3)
+    ms_pre, w = timed_steps(torch, dist, device, g_pre.replay, ksteps_p, args.warmup)
     windows.append(w)
+    last = {m["N"]: (m["name"], y) for m, y in zip(model, keep2[1])}   # each buffer holds its last writer's output
+    for name, y in last.values():
+        keep(f"prefill_{name}_last_layer", y[rows_p.to(device)])
     g_pe2e, hyp, h2dp, d2hp = plugin_graph(Mp, "gemm")
 
     def pe2e_step():
         g_pe2e.replay()
         torch.cuda.current_stream().synchronize()
         _ = float(hyp[0, 0])
-    ms_pe2e, w = timed_steps(torch, dist, device, pe2e_step, ksteps_p, 3)
+    ms_pe2e, w = timed_steps(torch, dist, device, pe2e_step, ksteps_p, args.warmup)
     windows.append(w)
+    keep("prefill_e2e_y", hyp[rows_p])
+    keep("prefill_rows", rows_p)
     # ---------------- decode end to end WITHOUT a graph (what an unmodified caller sees)
-    ms_eager, host_us, eager_kind, w = eager_e2e(1, min(args.steps, 100))
+    ms_eager, host_us, eager_kind, w = eager_e2e(1, args.steps)
     windows.append(w)
     sweep = batch_sweep() if (world == 1 and args.sweep) else None
     clocks = sampler.stop(windows)
@@ -382,10 +401,12 @@ def run_b200(args):
         del g_dec, g_e2e, g_pre, g_pe2e, keep1, keep2
         model.clear()
         torch.cuda.empty_cache()
-        tp = tp70b_measure(torch, dist, rank, world, device, min(args.steps, 100), args.warmup)
+        tp = tp70b_measure(torch, dist, rank, world, device, args.steps, args.warmup)
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, dump)
     step_ms = ms_dec / args.steps
     ach = bytes_step / (step_ms * 1e-3) / 1e9
     traffic = None
@@ -433,41 +454,31 @@ def run_b200(args):
         line["cpu_baseline"] = cpu_baseline(args.cpu_seconds)
     if world == 1 and args.ref_gpu:
         try:
-            line["reference_on_b200"] = reference_gpu(torch, model, make_inputs, device, min(args.steps, 200), lib)
+            line["reference_on_b200"] = reference_gpu(torch, model, make_inputs, device, args.steps, lib)
         except Exception as e:  # noqa: BLE001
             line["reference_on_b200"] = {"unavailable": repr(e)[:200]}
     print(json.dumps(line))
 
 
+def write_outputs(out_dir, arrays):
+    """DIR/<name>.npy, float32, for comparing two builds output for output (the inputs are seeded)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 def reference_wqlinears(torch, model, device, dtype):
-    """One reference-facing module per layer of `model`, sharing the layer's packed buffers: the reference's own
-    WQLinear (staged copy under baseline/_ref, see scripts/stage_reference.py) bound to this repo's plugin, else
-    this repo's mirror of it."""
+    """One reference-facing module per layer of `model`, sharing the layer's packed buffers: this repo's mirror of the
+    reference's WQLinear."""
     import llm_awq_b200 as P
     P.engine()
-    staged = os.path.join(ROOT, "baseline", "_ref")
-    cls, kind = None, "llm_awq_b200.WQLinear (mirror of the reference module)"
-    if os.path.exists(os.path.join(staged, "awq", "quantize", "qmodule.py")):
-        try:
-            if staged not in sys.path:
-                sys.path.insert(0, staged)
-            import contextlib
-            with contextlib.redirect_stdout(sys.stderr):   # the reference prints notices at import: stdout is the JSON line's
-                from awq.quantize.qmodule import WQLinear as RefWQLinear
-            cls, kind = RefWQLinear, "reference awq.quantize.qmodule.WQLinear (unmodified, baseline/_ref) on this plugin"
-        except Exception:  # noqa: BLE001
-            cls = None
     mods = []
     for m in model:
-        if cls is not None:
-            mod = cls(4, G, 128, 8, False, "cpu", dtype=dtype)   # tiny buffers, replaced below
-            mod.in_features, mod.out_features = m["K"], m["N"]
-        else:
-            mod = P.WQLinear(4, G, 128, 8, False, "cpu")
-            mod.in_features, mod.out_features = m["K"], m["N"]
+        mod = P.WQLinear(4, G, 128, 8, False, "cpu")   # tiny buffers, replaced below
+        mod.in_features, mod.out_features = m["K"], m["N"]
         mod.qweight, mod.scales, mod.scaled_zeros = m["qw"], m["sc"], m["sz"]
         mods.append(mod)
-    return mods, kind
+    return mods, "llm_awq_b200.WQLinear (mirror of the reference module)"
 
 
 def tp70b_measure(torch, dist, rank, world, device, steps, warmup):
@@ -718,7 +729,7 @@ def run_reference_gpu(args):
     def make_inputs(M, scale=1.0):
         g = torch.Generator(device=device).manual_seed(99 + M)
         return {K: (torch.randn(M, K, generator=g, device=device) * scale).to(torch.float16) for K in (4096, 14336)}
-    r = reference_gpu(torch, model, make_inputs, device, min(args.steps, 200))
+    r = reference_gpu(torch, model, make_inputs, device, args.steps)
     print(json.dumps({"impl": "reference-gpu", "metric": METRIC % 1, "value": r["decode"]["value"], "unit": UNIT, "n_gpus": 1,
                       "higher_is_better": True, "detail": r}))
 
@@ -726,17 +737,23 @@ def run_reference_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=500,
+                    help="timed steps of each GPU leg (the reference kernels' prefill comparison times 5; "
+                         "--impl reference times min(--steps, --cpu-steps) on the host)")
+    ap.add_argument("--warmup", type=int, default=10, help="untimed steps before each leg of --impl b200")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference", "reference-gpu"])
-    ap.add_argument("--prefill-steps", type=int, default=10)
+    ap.add_argument("--prefill-steps", type=int, default=None, help="timed prefill steps instead of --steps")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--cpu-steps", type=int, default=30)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-ref-gpu", dest="ref_gpu", action="store_false")
     ap.add_argument("--no-sweep", dest="sweep", action="store_false")
     ap.add_argument("--workload", default="llama3", choices=["llama3", "tp70b"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of each leg as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "llama3"):
+        ap.error("--dump-outputs writes the outputs of --impl b200 --workload llama3 only")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,8 +1,10 @@
 """Generate tests/golden/*.npz by running the REFERENCE's own Python on CPU.
 
-Run in the build container only (needs /root/reference; the GPU box does not have it):
+Needs a checkout of the reference (its path in AWQ_REFERENCE) and a built package:
 
     python tests/golden/make_golden.py
+
+reference_kernels.npz is made on a GPU from the reference's kernels instead (kernels_golden).
 
 The reference module ``awq.quantize.qmodule`` does ``import awq_inference_engine`` at
 import time (qmodule.py:4); a stub module is registered for that name because only the
@@ -214,6 +216,174 @@ def mlp_callsite_golden():
     print("wrote reference_mlp_callsite.npz", len(out), "arrays")
 
 
+def callsites_golden():
+    """tests/golden/reference_callsites.npz: the reference's own, unmodified call sites EXECUTED on CPU over a stub
+    ``awq_inference_engine`` whose linears are the W4A16 oracle rounded to the element type, on the inputs of
+    tests/test_reference_callsites_gpu.py (regenerated there from the same seeds):
+      * awq.quantize.qmodule.WQLinear                the state dict of a 256 -> 64 layer; forward (qmodule.py:201-224):
+                                                     which entry it calls, the bias added to the rounded output
+      * tinychat.modules.fused_mlp.QuantLlamaMLP     our_llama_mlp (fused_mlp.py:36-83), both branches
+      * tinychat.modules.fused_attn.make_quant_attn  the fused QKV WQLinear it builds (fused_attn.py:566-594): shapes and
+                                                     sums of its buffers, and its outputs
+    Outputs are stored at up to 4 seeded rows (callsite_rows) and every other column, as bit patterns of the element
+    type."""
+    root = os.path.dirname(os.path.dirname(HERE))
+    for p in (root, os.path.join(root, "tests"), REF):
+        if p not in sys.path:
+            sys.path.insert(0, p)
+    from oracle import w4a16_oracle as O
+    from awq_testutil import gen_layer, gen_x
+    from test_reference_callsites_gpu import MLP_TOKENS, QKV_TOKENS, WQ_SHAPES, callsite_rows, layer_bias
+    # the one stub every reference module imported in this process holds: generators that ran before bound their own
+    # entries onto it, so this one rebinds them rather than registering a second stub those modules would not see
+    eng = sys.modules.setdefault("awq_inference_engine", types.ModuleType("awq_inference_engine"))
+    calls = []
+
+    def linear(x, qw, s, z):
+        tag = "f16" if x.dtype == torch.float16 else "bf16"
+        x2 = x.reshape(-1, x.shape[-1]).double().numpy()
+        y = O.wq_linear_forward(x2, qw.numpy(), s.double().numpy(), z.double().numpy(), dtype=tag)
+        return torch.from_numpy(O.rounder(tag)(y)).to(x.dtype).reshape(*x.shape[:-1], -1)
+
+    def gemv(x, qw, s, z, m, n, k, g):
+        calls.append("gemv")
+        return linear(x, qw, s, z)
+
+    def gemm(x, qw, s, z):
+        calls.append("gemm")
+        return linear(x, qw, s, z)
+    eng.gemv_forward_cuda_new, eng.gemm_forward_cuda_new = gemv, gemm
+    import contextlib
+    with contextlib.redirect_stdout(sys.stderr):
+        import awq.quantize.qmodule as qmodule
+        import tinychat.utils.constants as constants
+        constants.init()
+        import tinychat.modules.fused_mlp as fused_mlp
+        import tinychat.modules.fused_attn as fused_attn
+
+    def ref_wqlinear(K, N, dtype, seed, bias=False):
+        m = qmodule.WQLinear(4, 128, K, N, bias, "cpu", dtype=dtype)
+        m.qweight, m.scales, m.scaled_zeros = gen_layer(N, K, dtype, seed=seed)
+        if bias:
+            m.bias = layer_bias(N, dtype, seed)
+        return m
+    bits = lambda t, M: t.reshape(M, -1)[callsite_rows(M)][:, ::2].contiguous().view(torch.int16).numpy()
+    out = {}
+    for k, v in qmodule.WQLinear(4, 128, 256, 64, False, "cpu").state_dict().items():   # the module's buffers
+        out[f"state_{k}_shape"], out[f"state_{k}_dtype"] = np.array(v.shape), np.array(str(v.dtype))
+    K, N = 1024, 768
+    for tag, dt in (("f16", torch.float16), ("bf16", torch.bfloat16)):
+        for bias in (False, True):
+            m = ref_wqlinear(K, N, dt, 5, bias)
+            for shape in WQ_SHAPES:
+                M = shape[0] * shape[1]
+                x = gen_x(M, K, dt, seed=shape[1]).view(*shape, K)
+                del calls[:]
+                y = m(x)
+                key = f"wq_{tag}_b{int(bias)}_{shape[0]}x{shape[1]}"
+                out[key + "_y"] = bits(y, M)
+                out[key + "_calls"] = np.array(calls)
+    dt, H, I = torch.float16, 1024, 2816
+    gate, up, down = ref_wqlinear(H, I, dt, 11), ref_wqlinear(H, I, dt, 12), ref_wqlinear(I, H, dt, 13)
+    mlp = fused_mlp.QuantLlamaMLP(gate, down, up)
+    for tokens in MLP_TOKENS:
+        x = (gen_x(tokens, H, dt, seed=tokens) * 0.5).view(1, tokens, H)
+        del calls[:]
+        c = mlp.our_llama_mlp(x)
+        out[f"mlp_t{tokens}_c"] = bits(c, tokens)
+        out[f"mlp_t{tokens}_calls"] = np.array(calls)
+    H, KV = 1024, 256
+
+    class LlamaAttentionFused(torch.nn.Module):   # the class NAME is what make_quant_attn matches (:559-563)
+        def __init__(self):
+            super().__init__()
+            self.q_proj, self.k_proj = ref_wqlinear(H, H, dt, 21), ref_wqlinear(H, KV, dt, 22)
+            self.v_proj, self.o_proj = ref_wqlinear(H, KV, dt, 23), ref_wqlinear(H, H, dt, 24)
+            self.args = types.SimpleNamespace(hidden_size=H, num_attention_heads=8, num_key_value_heads=2,
+                                              max_position_embeddings=128, rope_theta=10000.0, rope_scaling=None)
+            self.kv_max_seq_len = 64
+
+    class Holder(torch.nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.attn = LlamaAttentionFused()
+    model = Holder()
+    with contextlib.redirect_stdout(sys.stderr):
+        fused_attn.make_quant_attn(model, "cpu")
+    qkv = model.attn.qkv_proj
+    for nm in ("qweight", "scales", "scaled_zeros"):
+        t = getattr(qkv, nm)
+        out[f"qkv_{nm}_shape"] = np.array(t.shape)
+        out[f"qkv_{nm}_sum"] = t.float().numpy().astype(np.float64).sum() if t.is_floating_point() else t.numpy().astype(np.int64).sum()
+    for tokens in QKV_TOKENS:
+        x = gen_x(tokens, H, dt, seed=30 + tokens).view(1, tokens, H)
+        del calls[:]
+        y = qkv(x)
+        out[f"qkv_t{tokens}_y"] = bits(y, tokens)
+        out[f"qkv_t{tokens}_calls"] = np.array(calls)
+    np.savez_compressed(os.path.join(HERE, "reference_callsites.npz"), **out)
+    print("wrote reference_callsites.npz", len(out), "arrays")
+
+
+def kernels_golden(out_dir=HERE):
+    """tests/golden/reference_kernels.npz: what the reference's own CUDA kernels, rebuilt for sm_100a by
+    oracle/build_ref.py, return on the inputs of the GPU tests that compare against them.  Needs a CUDA device and
+    oracle/_ref (run it where both exist):
+
+        python tests/golden/make_golden.py --kernels [OUT_DIR]
+
+    Stored (samples keep the file small; the tests regenerate the inputs from the same seeds):
+      * W4A16 GEMV / GEMM (tests/test_gpu_parity.py::test_matches_reference_kernels): bit patterns of y at up to 16
+        seeded rows and at the output columns 0, 74, 148, ..., plus the sums of x and qweight that identify the inputs
+      * layernorm_forward_cuda (tests/test_layer_ops_gpu.py): bit patterns of 8192 seeded elements of the output
+      * rotary_embedding_neox (tests/test_zz_rope_neox_gpu.py): bit patterns of 64 seeded (token, head) rows of q
+        and of k after the in-place rotation"""
+    root = os.path.dirname(os.path.dirname(HERE))
+    for p in (root, os.path.join(root, "tests"), os.path.join(root, "oracle", "_ref")):
+        if p not in sys.path:
+            sys.path.insert(0, p)
+    import ref_awq_engine as ref
+    from awq_testutil import gen_layer, gen_x
+    from test_gpu_parity import REF_KERNEL_CASES, ref_kernel_rows
+    from test_layer_ops_gpu import rmsnorm_ref_inputs
+    from test_zz_rope_neox_gpu import rope_ref_inputs
+    dev = "cuda:0"
+    out = {}
+    for M, N, K in REF_KERNEL_CASES:
+        for tag, dt in (("f16", torch.float16), ("bf16", torch.bfloat16)):
+            qw, s, z = gen_layer(N, K, dt, seed=9, device=dev)
+            x = (gen_x(M, K, dt, seed=10, device=dev) * 0.25).contiguous()
+            if M < 8:
+                y = ref.gemv_forward_cuda_new(x, qw, s, z, M, N, K, 128)
+            else:
+                y = ref.gemm_forward_cuda_new(x, qw, s, z)
+            torch.cuda.synchronize()
+            key = f"w4_{M}x{N}x{K}_{tag}"
+            out[key + "_y"] = y.cpu()[ref_kernel_rows(M)][:, ::74].contiguous().view(torch.int16).numpy()
+            out[key + "_xsum"] = np.float64(x.float().cpu().numpy().astype(np.float64).sum())
+            out[key + "_qwsum"] = np.int64(qw.cpu().numpy().astype(np.int64).sum())
+    pick = np.random.default_rng(7)
+    for tag, dt in (("f16", torch.float16), ("bf16", torch.bfloat16)):
+        x, gamma = rmsnorm_ref_inputs(dt, dev)
+        y = torch.empty_like(x)
+        ref.layernorm_forward_cuda(x, gamma, y, 1e-6)
+        torch.cuda.synchronize()
+        idx = np.sort(pick.choice(y.numel(), 32768, replace=False))[::4].astype(np.int32)
+        out[f"rms_{tag}_idx"] = idx
+        out[f"rms_{tag}_y"] = y.view(torch.int16).cpu().reshape(-1).numpy()[idx]
+        pos, q, k, cache = rope_ref_inputs(dt, dev)
+        ref.rotary_embedding_neox(pos, q, k, q.shape[-1], cache)
+        torch.cuda.synchronize()
+        for nm, t in (("q", q), ("k", k)):
+            rows = t.reshape(-1, t.shape[-1])
+            idx = np.sort(pick.choice(rows.shape[0], 256, replace=False))[::4].astype(np.int32)
+            out[f"rope_{tag}_{nm}_idx"] = idx
+            out[f"rope_{tag}_{nm}"] = rows.view(torch.int16).cpu().numpy()[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.savez_compressed(os.path.join(out_dir, "reference_kernels.npz"), **out)
+    print("wrote reference_kernels.npz", len(out), "arrays")
+
+
 def main():
     qmodule, pseudo_quantize_tensor = _import_reference()
     g = torch.Generator().manual_seed(20260922)
@@ -291,7 +461,12 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
-    repacker_golden()
-    layer_ops_golden()
-    mlp_callsite_golden()
+    if "--kernels" in sys.argv:
+        rest = sys.argv[sys.argv.index("--kernels") + 1:]
+        kernels_golden(rest[0] if rest else HERE)
+    else:
+        main()
+        repacker_golden()
+        layer_ops_golden()
+        mlp_callsite_golden()
+        callsites_golden()

@@ -115,23 +115,22 @@ def test_oracle_is_not_imported_by_the_product():
                 assert "oracle" not in open(os.path.join(dirpath, f)).read().replace("test oracle", ""), f
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/awq"), reason="reference checkout only exists in the build container")
 def test_unmodified_reference_wqlinear_binds_to_this_engine():
     """The reference's own qmodule.py does `import awq_inference_engine` (qmodule.py:4): with our plugin
-    directory on sys.path it must pick up THIS build, and its WQLinear.forward must reach our entry points
-    (which reject CPU tensors instead of computing on the host)."""
-    import importlib.util
+    directory on sys.path that import must pick up THIS build; the drop-in WQLinear must hold the buffers the reference's
+    WQLinear holds (stored in tests/golden/reference_callsites.npz; the reference's code does not run here), and its
+    forward must reach our entry points (which reject CPU tensors instead of computing on the host)."""
+    import importlib
     import sys
     P.install()
     sys.modules.pop("awq_inference_engine", None)
-    spec = importlib.util.spec_from_file_location("ref_qmodule_live", "/root/reference/awq/quantize/qmodule.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    assert os.path.abspath(ref.awq_inference_engine.__file__).startswith(P.install())
-    m = ref.WQLinear(4, 128, 256, 64, False, "cpu")
-    ours = P.WQLinear(4, 128, 256, 64, False, "cpu")
-    assert {k: (v.shape, v.dtype) for k, v in m.state_dict().items()} == \
-           {k: (v.shape, v.dtype) for k, v in ours.state_dict().items()}
+    eng = importlib.import_module("awq_inference_engine")
+    assert os.path.abspath(eng.__file__).startswith(P.install())
+    gold = np.load(os.path.join(ROOT, "tests", "golden", "reference_callsites.npz"))
+    want = {k[len("state_"):-len("_shape")]: (tuple(gold[k]), str(gold[k[:-len("_shape")] + "_dtype"]))
+            for k in gold.files if k.startswith("state_") and k.endswith("_shape")}
+    m = P.WQLinear(4, 128, 256, 64, False, "cpu")
+    assert {k: (tuple(v.shape), str(v.dtype)) for k, v in m.state_dict().items()} == want
     for tokens in (1, 9):      # GEMV branch and GEMM branch of the reference's forward (qmodule.py:206-220)
         with pytest.raises(RuntimeError, match="CUDA"):
             m(torch.zeros(tokens, 256, dtype=torch.float16))

@@ -1,6 +1,4 @@
-"""The reference's OWN call sites, unmodified, running on this repo's `awq_inference_engine` plugin on the GPU
-(SURVEY.md §8 a13, a3; VERDICT r1 item 2a).  `scripts/stage_reference.py` copies the reference's Python packages
-byte-for-byte into the git-ignored baseline/_ref/ (the GPU box has no /root/reference); this file imports
+"""The reference's OWN call sites and what they compute, against this repo's modules on the GPU (SURVEY.md §8 a13, a3):
 
     awq.quantize.qmodule.WQLinear                  forward: qmodule.py:201-224 (GEMV for < 8 tokens, else GEMM, + bias)
     tinychat.modules.fused_mlp.QuantLlamaMLP       our_llama_mlp: fused_mlp.py:36-83 (both branches, incl. the GEMM
@@ -8,19 +6,19 @@ byte-for-byte into the git-ignored baseline/_ref/ (the GPU box has no /root/refe
     tinychat.modules.fused_attn.make_quant_attn    the fused-QKV WQLinear built by concatenating packed tensors,
                                                    fused_attn.py:566-594
 
-from there with `awq_inference_engine` resolving to llm_awq_b200/plugin, and checks every result against the CPU
-oracle.  Nothing of the reference is modified or monkey-patched."""
-import hashlib
-import json
+tests/golden/reference_callsites.npz holds what those call sites, unmodified, returned when executed on CPU over
+oracle-backed engine calls, and which engine entry each made (tests/golden/make_golden.py::callsites_golden), on the
+inputs regenerated here from the same seeds.  The repo's drop-ins (llm_awq_b200.WQLinear, llm_awq_b200.fused_mlp.
+QuantLlamaMLP with the reference's GEMM-branch zeros) must make the same entry calls on the plugin and return the same
+results; every result is also checked against the CPU oracle."""
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
 import llm_awq_b200 as P
+from llm_awq_b200.fused_mlp import QuantLlamaMLP
 from oracle import layer_oracle as LO
 from oracle import w4a16_oracle as O
 from awq_testutil import dt_name, gen_layer, gen_x, np64, oracle_forward, rel_err
@@ -28,72 +26,95 @@ from test_gpu_parity import check
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-STAGED = os.path.join(ROOT, "baseline", "_ref")
+WQ_SHAPES = [(1, 1), (1, 7), (1, 8), (2, 40), (1, 300)]
+MLP_TOKENS = [1, 4, 7, 8, 64, 300]
+QKV_TOKENS = [1, 5, 16, 130]
+
+
+def callsite_rows(M):
+    """Rows of an [M, N] output kept in the golden file (at every other column): all of them up to 4, else 4 seeded
+    ones."""
+    return np.arange(M) if M <= 4 else np.sort(np.random.default_rng(M).choice(M, 4, replace=False))
+
+
+def layer_bias(N, dtype, seed):
+    g = torch.Generator().manual_seed(seed + 1)
+    return (torch.randn(N, generator=g) * 0.1).to(dtype)
 
 
 @pytest.fixture(scope="module")
-def ref():
-    """The staged reference packages, importable, with the plugin as `awq_inference_engine`."""
-    man = os.path.join(STAGED, "MANIFEST.json")
-    assert os.path.exists(man), "run scripts/stage_reference.py in the build container (baseline/_ref/ travels with gpurun)"
-    files = json.load(open(man))["files"]
-    for rel in ("awq/quantize/qmodule.py", "tinychat/modules/fused_mlp.py", "tinychat/modules/fused_attn.py"):
-        assert hashlib.sha256(open(os.path.join(STAGED, rel), "rb").read()).hexdigest() == files[rel], rel + " was modified"
-    eng = P.engine()                       # puts llm_awq_b200/plugin on sys.path and imports the extension
-    assert sys.modules["awq_inference_engine"] is eng
-    if STAGED not in sys.path:
-        sys.path.insert(0, STAGED)
-    import awq.quantize.qmodule as qmodule
-    import tinychat.utils.constants as constants
-    constants.init()                        # tinychat/demo.py and benchmark.py do this before importing the modules
-    import tinychat.modules.fused_mlp as fused_mlp
-    import tinychat.modules.fused_attn as fused_attn
-    assert qmodule.awq_inference_engine is eng and fused_mlp.awq_inference_engine is eng
-    assert os.path.realpath(qmodule.__file__).startswith(os.path.realpath(STAGED))
-    return types.SimpleNamespace(qmodule=qmodule, fused_mlp=fused_mlp, fused_attn=fused_attn)
+def gold():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_callsites.npz"))
 
 
-def _ref_wqlinear(ref, K, N, dtype, seed, bias=False):
-    """A reference WQLinear with synthetic packed buffers (the constructor zero-fills them, qmodule.py:98-137)."""
-    m = ref.qmodule.WQLinear(4, 128, K, N, bias, DEV, dtype=dtype)
+def _wqlinear(K, N, dtype, seed, bias=False):
+    """A WQLinear with synthetic packed buffers (the constructor zero-fills them, qmodule.py:98-137)."""
+    m = P.WQLinear(4, 128, K, N, bias, DEV, dtype=dtype)
     qw, s, z = gen_layer(N, K, dtype, seed=seed, device=DEV)
     assert m.qweight.shape == qw.shape and m.scales.shape == s.shape and m.scaled_zeros.shape == z.shape
     m.qweight, m.scales, m.scaled_zeros = qw, s, z
     if bias:
-        g = torch.Generator().manual_seed(seed + 1)
-        m.bias = (torch.randn(N, generator=g) * 0.1).to(dtype).to(DEV)
+        m.bias = layer_bias(N, dtype, seed).to(DEV)
     return m
 
 
+def _entries(gold, key, tokens):
+    """The reference made one engine call per linear, the GEMV entry below 8 tokens and the GEMM entry from 8."""
+    calls = [str(c) for c in gold[key + "_calls"]]
+    assert set(calls) == {"gemv" if tokens < 8 else "gemm"}
+    return len(calls)
+
+
+def _sample(y, M):
+    return np64(y.reshape(M, -1))[callsite_rows(M)][:, ::2]
+
+
+def _stored(gold, key, dtype):
+    return np64(torch.from_numpy(gold[key]).view(dtype))
+
+
 @pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16], ids=["f16", "bf16"])
-@pytest.mark.parametrize("shape", [(1, 1), (1, 7), (1, 8), (2, 40), (1, 300)], ids=str)
+@pytest.mark.parametrize("shape", WQ_SHAPES, ids=str)
 @pytest.mark.parametrize("bias", [False, True])
-def test_unmodified_reference_wqlinear_forward(ref, shape, dtype, bias):
+def test_unmodified_reference_wqlinear_forward(gold, shape, dtype, bias):
+    """llm_awq_b200.WQLinear.forward against what the reference's unmodified WQLinear.forward returned (stored): the same
+    engine entry, one launch, the same output; the reference's code does not run here."""
     K, N = 1024, 768
-    m = _ref_wqlinear(ref, K, N, dtype, seed=5, bias=bias)
-    x = gen_x(shape[0] * shape[1], K, dtype, seed=shape[1], device=DEV).view(*shape, K)
+    M = shape[0] * shape[1]
+    key = f"wq_{dt_name(dtype)}_b{int(bias)}_{shape[0]}x{shape[1]}"
+    m = _wqlinear(K, N, dtype, seed=5, bias=bias)
+    x = gen_x(M, K, dtype, seed=shape[1], device=DEV).view(*shape, K)
     before = P.engine().launch_count()
-    y = m(x)                                                    # qmodule.py:201-224, unmodified
+    y = m(x)
     torch.cuda.synchronize()
-    assert P.engine().launch_count() == before + 1 and y.shape == (*shape, N)
+    assert P.engine().launch_count() == before + _entries(gold, key, M) and y.shape == (*shape, N)
     want = oracle_forward(x.view(-1, K), m.qweight, m.scales, m.scaled_zeros, dtype)
     if bias:
         want = O.rounder(dt_name(dtype))(want) + np64(m.bias)   # the reference adds the bias to the ROUNDED output (:221)
-    check(y.view(-1, N), want, dtype, tol=1e-3 if not bias else (1e-3 if dtype == torch.float16 else 6e-3))
+    tol = 1e-3 if not bias else (1e-3 if dtype == torch.float16 else 6e-3)
+    check(y.view(-1, N), want, dtype, tol=tol)
+    assert rel_err(_sample(y, M), _stored(gold, key + "_y", dtype)) <= tol
 
 
-@pytest.mark.parametrize("tokens", [1, 4, 7, 8, 64, 300])
-def test_unmodified_reference_fused_mlp_both_branches(ref, tokens):
+@pytest.mark.parametrize("tokens", MLP_TOKENS)
+def test_unmodified_reference_fused_mlp_both_branches(gold, tokens):
     """QuantLlamaMLP.our_llama_mlp: < 8 tokens -> two GEMV calls with the zeros as stored (fused_mlp.py:40-60);
     otherwise two GEMM calls with `scaled_zeros - 8 * scales` (:65-77; the tensor expression is evaluated in fp16 by
-    torch before the call, and the oracle is given exactly that tensor: "use the zeros you are given")."""
+    torch before the call, and the oracle is given exactly that tensor: "use the zeros you are given").  The reference's
+    code does not run here: its stored output is compared with the drop-in llm_awq_b200.fused_mlp.QuantLlamaMLP, which
+    makes one engine call of the fused front half in place of the reference's two linears + F.silu + multiply.  That
+    call launches the one-kernel gate+up+SiLU*mul for one token, else the reference's linears (one launch each) and one
+    SiLU*mul kernel."""
     dtype, H, I = torch.float16, 1024, 2816
-    gate, up, down = (_ref_wqlinear(ref, H, I, dtype, 11), _ref_wqlinear(ref, H, I, dtype, 12), _ref_wqlinear(ref, I, H, dtype, 13))
-    mlp = ref.fused_mlp.QuantLlamaMLP(gate, down, up)
+    gate, up, down = _wqlinear(H, I, dtype, 11), _wqlinear(H, I, dtype, 12), _wqlinear(I, H, dtype, 13)
+    mlp = QuantLlamaMLP(gate, down, up, legacy_gemm_zero_offset=True)
+    ref_calls = _entries(gold, f"mlp_t{tokens}", tokens)
+    assert ref_calls == 2                                        # gate_proj and up_proj
     x = (gen_x(tokens, H, dtype, seed=tokens, device=DEV) * 0.5).view(1, tokens, H)
-    c = mlp.our_llama_mlp(x)                                     # unmodified
+    before = P.engine().launch_count()
+    c = mlp.our_llama_mlp(x)
     torch.cuda.synchronize()
+    assert P.engine().launch_count() - before == (1 if tokens == 1 else ref_calls + 1)
     assert c.shape == (1, tokens, I)
     if tokens < 8:
         gz, uz = gate.scaled_zeros, up.scaled_zeros
@@ -103,40 +124,36 @@ def test_unmodified_reference_fused_mlp_both_branches(ref, tokens):
                         (up.qweight.cpu().numpy(), np64(up.scales), np64(uz)), dtype="f16")
     # products of two rounded factors: 2 ulp of fp16 normwise
     assert rel_err(np64(c.view(tokens, I)), want) < 1.5e-3
+    assert rel_err(_sample(c, tokens), _stored(gold, f"mlp_t{tokens}_c", dtype)) < 1.5e-3
     y = mlp(x)                                                   # + down_proj through WQLinear.forward
     torch.cuda.synchronize()
     want_y = oracle_forward(c.view(tokens, I), down.qweight, down.scales, down.scaled_zeros, dtype)
     check(y.view(tokens, H), want_y, dtype)
 
 
-def test_unmodified_reference_make_quant_attn_concatenation(ref):
-    """make_quant_attn (fused_attn.py:556-640) on a module that looks like tinychat's LlamaAttentionFused: the fused
-    QKV layer it builds by torch.cat of qweight (dim 0) / scales / scaled_zeros (dim 1) must give [q; k; v] of the three
-    separate projections, through the plugin, for decode and prefill token counts."""
+def test_unmodified_reference_make_quant_attn_concatenation(gold):
+    """make_quant_attn (fused_attn.py:556-640) builds the fused QKV layer by torch.cat of qweight (dim 0) / scales /
+    scaled_zeros (dim 1): the same concatenation here must give the buffers the reference built (stored shapes and
+    sums), and [q; k; v] of the three separate projections through the plugin, as the reference's fused layer returned
+    them, for decode and prefill token counts.  The reference's code does not run here."""
     dtype, H, KV = torch.float16, 1024, 256
-
-    class LlamaAttentionFused(torch.nn.Module):   # the class NAME is what make_quant_attn matches (:559-563)
-        def __init__(self):
-            super().__init__()
-            self.q_proj, self.k_proj = _ref_wqlinear(ref, H, H, dtype, 21), _ref_wqlinear(ref, H, KV, dtype, 22)
-            self.v_proj, self.o_proj = _ref_wqlinear(ref, H, KV, dtype, 23), _ref_wqlinear(ref, H, H, dtype, 24)
-            self.args = types.SimpleNamespace(hidden_size=H, num_attention_heads=8, num_key_value_heads=2,
-                                              max_position_embeddings=128, rope_theta=10000.0, rope_scaling=None)
-            self.kv_max_seq_len = 64
-
-    class Holder(torch.nn.Module):
-        def __init__(self):
-            super().__init__()
-            self.attn = LlamaAttentionFused()
-
-    model = Holder()
-    parts = [(m.qweight.clone(), m.scales.clone(), m.scaled_zeros.clone()) for m in (model.attn.q_proj, model.attn.k_proj, model.attn.v_proj)]
-    ref.fused_attn.make_quant_attn(model, DEV)                   # unmodified; replaces model.attn
-    qkv = model.attn.qkv_proj
-    assert type(qkv) is ref.qmodule.WQLinear and qkv.out_features == H + 2 * KV
-    for tokens in (1, 5, 16, 130):
+    parts = [_wqlinear(H, H, dtype, 21), _wqlinear(H, KV, dtype, 22), _wqlinear(H, KV, dtype, 23)]
+    qkv = P.WQLinear(4, 128, H, H + 2 * KV, False, DEV, dtype=dtype)
+    qkv.qweight = torch.cat([p.qweight for p in parts], dim=0)
+    qkv.scales = torch.cat([p.scales for p in parts], dim=1).contiguous()
+    qkv.scaled_zeros = torch.cat([p.scaled_zeros for p in parts], dim=1).contiguous()
+    for nm in ("qweight", "scales", "scaled_zeros"):
+        t = getattr(qkv, nm).cpu()
+        assert tuple(t.shape) == tuple(gold[f"qkv_{nm}_shape"])
+        s = t.float().numpy().astype(np.float64).sum() if t.is_floating_point() else t.numpy().astype(np.int64).sum()
+        assert s == gold[f"qkv_{nm}_sum"], nm
+    for tokens in QKV_TOKENS:
+        key = f"qkv_t{tokens}"
         x = gen_x(tokens, H, dtype, seed=30 + tokens, device=DEV).view(1, tokens, H)
+        before = P.engine().launch_count()
         y = qkv(x)
         torch.cuda.synchronize()
-        want = np.concatenate([oracle_forward(x.view(tokens, H), *p, dtype) for p in parts], axis=1)
+        assert P.engine().launch_count() == before + _entries(gold, key, tokens)
+        want = np.concatenate([oracle_forward(x.view(tokens, H), p.qweight, p.scales, p.scaled_zeros, dtype) for p in parts], axis=1)
         check(y.view(tokens, -1), want, dtype)
+        assert rel_err(_sample(y, tokens), _stored(gold, key + "_y", dtype)) <= 1e-3

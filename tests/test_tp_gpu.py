@@ -1,4 +1,4 @@
-"""Tensor-parallel modules on real kernels + NCCL (needs >= 2 GPUs; `gpurun --gpus 2`)."""
+"""Tensor-parallel modules on real kernels + NCCL (needs >= 2 GPUs)."""
 import os
 
 import numpy as np

@@ -1,6 +1,6 @@
 """GPU parity of `rotary_embedding_neox` (in-place NeoX RoPE from a cos|sin table; the HF-attention branch of tinychat,
 tinychat/modules/fused_attn.py:61-79) through the C ABI and the `awq_inference_engine` plugin, against
-oracle/layer_oracle.py and -- when present -- the reference's own kernel rebuilt for sm_100a (oracle/_ref).
+oracle/layer_oracle.py and the stored output of the reference's own kernel rebuilt for sm_100a (tests/golden).
 
 Tolerances: the kernel rounds ONCE to the element type from fp32 products, so against the float64 oracle an element
 is equal or one ulp off; the reference's kernel multiplies and adds in the element type (up to three roundings per
@@ -10,7 +10,6 @@ The kernel's body is also checked without a GPU (tests/test_rope_neox_host.py). 
 is the newest entry of the plugin."""
 import ctypes
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -23,17 +22,6 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 DTYPES = [torch.float16, torch.bfloat16]
 ULP = {torch.float16: 2.0 ** -10, torch.bfloat16: 2.0 ** -7}
-
-
-def _ref_engine():
-    d = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-    if d not in sys.path:
-        sys.path.insert(0, d)
-    try:
-        import ref_awq_engine
-    except ImportError:
-        return None
-    return ref_awq_engine if hasattr(ref_awq_engine, "rotary_embedding_neox") else None
 
 
 def _inputs(tokens, qh, kh, hs, rot, dtype, seed, maxpos=211):
@@ -162,23 +150,30 @@ def test_views_into_a_fused_qkv_buffer_and_graph_replay():
     assert torch.equal(dbuf[:, (qh + kh) * hs:].cpu(), buf[:, (qh + kh) * hs:])
 
 
-@pytest.mark.parametrize("dtype", DTYPES, ids=["f16", "bf16"])
-def test_vs_reference_kernel(dtype):
-    ref = _ref_engine()
-    if ref is None:
-        pytest.skip("oracle/_ref without rotary_embedding_neox (built by oracle/build_ref.py in the build container)")
-    eng = P.engine()
+def rope_ref_inputs(dtype, device):
+    """pos [1, 33], q and k [1, 33, 1, 32, 128] and the cos|sin table of test_vs_reference_kernel, on `device`; the
+    reference kernel's in-place result on them is stored in tests/golden/reference_kernels.npz
+    (tests/golden/make_golden.py --kernels)."""
     b, t, H, D = 1, 33, 32, 128
     pos, q, k, cache = _inputs(b * t, H, H, D, D, dtype, seed=21)
-    mine_q, mine_k = q.view(b, t, 1, H, D).to(DEV), k.view(b, t, 1, H, D).to(DEV)
-    ref_q, ref_k = mine_q.clone(), mine_k.clone()
-    dpos, dcache = pos.view(b, t).to(DEV), cache.to(DEV)
-    eng.rotary_embedding_neox(dpos, mine_q, mine_k, D, dcache)
-    ref.rotary_embedding_neox(dpos, ref_q, ref_k, D, dcache)
+    return pos.view(b, t).to(device), q.view(b, t, 1, H, D).to(device), k.view(b, t, 1, H, D).to(device), cache.to(device)
+
+
+@pytest.mark.parametrize("dtype", DTYPES, ids=["f16", "bf16"])
+def test_vs_reference_kernel(dtype):
+    eng = P.engine()
+    dpos, mine_q, mine_k, dcache = rope_ref_inputs(dtype, DEV)
+    q, k = mine_q.cpu(), mine_k.cpu()
+    eng.rotary_embedding_neox(dpos, mine_q, mine_k, mine_q.shape[-1], dcache)
     torch.cuda.synchronize()
-    for a, r, x in ((mine_q, ref_q, q), (mine_k, ref_k, k)):
-        a64, r64 = a.double().cpu().view(b * t, H, D), r.double().cpu().view(b * t, H, D)
-        scale = x.double().abs().amax(dim=-1, keepdim=True)               # |x'| <= |x| + |y| <= 2 max|head|
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_kernels.npz"))
+    tag = "f16" if dtype == torch.float16 else "bf16"
+    for nm, a, x in (("q", mine_q, q), ("k", mine_k, k)):
+        idx = torch.from_numpy(gold[f"rope_{tag}_{nm}_idx"]).long()
+        D = x.shape[-1]
+        r64 = torch.from_numpy(gold[f"rope_{tag}_{nm}"]).view(dtype).double()
+        a64 = a.cpu().reshape(-1, D)[idx].double()
+        scale = x.reshape(-1, D)[idx].double().abs().amax(dim=-1, keepdim=True)   # |x'| <= |x| + |y| <= 2 max|head|
         assert bool(((a64 - r64).abs() <= 4 * ULP[dtype] * scale).all())
         num, den = (a64 - r64).norm(dim=-1), r64.norm(dim=-1)
         assert bool((num <= 2 * ULP[dtype] * den).all())
