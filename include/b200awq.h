@@ -130,7 +130,9 @@ int b200awq_rmsnorm(const void* x, const void* gamma, void* y, int m, int n, flo
  * step's q and k are rotated at position t = length_per_sample ? length_per_sample[b] : timestep (angle t * scale /
  * base^(2i / rotary_dim); neox != 0 pairs (i, i + rotary_dim / 2), else (2i, 2i + 1)) and rounded to the element type;
  * k and v are stored at cache slot t % max_len; out = softmax(q K^T / sqrt(head_dim)) V over the last min(t + 1,
- * max_len) positions.  heads / kv_heads must be 1, 2, 4 or 8, head_dim a multiple of 8 up to 256 that divides 2048.
+ * max_len) positions.  G = heads / kv_heads is any integer from 1 to 128 (query head h reads KV head h / G).
+ * head_dim: a multiple of 8 up to 256 for G <= 8, a multiple of 16 up to 256 for G > 8 (every head dim the reference
+ * accepts); other shapes return B200AWQ_ERR_SHAPE.
  * `workspace`: >= b200awq_single_query_attention_workspace_bytes(...) bytes of device memory, ZERO before the first
  * use, then owned by the kernels (they leave it zero where it matters); one workspace per stream.  ALiBi is not
  * supported (the reference's alibi_slopes argument must be None). */

@@ -148,7 +148,9 @@ void layernorm_forward_cuda(torch::Tensor _input, torch::Tensor _gamma, torch::T
 }
 
 // reference: awq/kernels/csrc/attention/ft_attention.cpp:112-184 (same checks, same argument order and defaults,
-// pybind.cpp:24-27).  alibi_slopes must be None; fp32 tensors are not dispatched.
+// pybind.cpp:24-27).  Any nheads / nheads_kv ratio up to 128 (the GQA / multi-query callers of Qwen2, Llama-3.2,
+// Falcon); the head_dim limits are those of b200awq_single_query_attention.  alibi_slopes must be None; fp32 tensors are
+// not dispatched.
 torch::Tensor single_query_attention(const torch::Tensor q, const torch::Tensor k, const torch::Tensor v, torch::Tensor k_cache,
                                      torch::Tensor v_cache, c10::optional<const torch::Tensor> length_per_sample_,
                                      c10::optional<const torch::Tensor> alibi_slopes_, const int timestep,

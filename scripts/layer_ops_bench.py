@@ -82,4 +82,38 @@ for L, t in ((2048, 2047), (8192, 8191)):
     b = 2 * (t + 1) * D * 2 * Hkv
     out["attention_ctx%d" % (t + 1)] = {"us": round(us, 3), "GBs": round(b / us / 1e3, 1), "hbm_frac": round(b / us / 1e3 / peaks["hbm"], 3),
                                         "kv_bytes": b}
+
+# ---- decode attention at other query-to-KV head ratios G = H / Hkv: the CUDA-core kernel (G <= 8) and the tensor-core
+# kernel (G > 8).  Enough caches per graph to stream >= 384 MB (3x L2) per replay; one launch per cache.
+for name, H, Hkv, D, batches in (("qwen2_7b", 28, 4, 128, (1,)), ("qwen2_1p5b", 12, 2, 128, (1,)),
+                                  ("g16", 128, 8, 64, (1, 8)), ("mqa71", 71, 1, 64, (1, 8))):
+    G = H // Hkv
+    for B in batches:
+        for L in (2048, 8192):
+            t = L - 1
+            b = 2 * B * (t + 1) * D * 2 * Hkv
+            n = max(4, min(512, -(-(384 << 20) // b)))
+            kcs = [torch.randn(B, Hkv, D // 8, L, 8, device=dev).half() for _ in range(n)]
+            vcs = [torch.randn(B, Hkv, L, D, device=dev).half() for _ in range(n)]
+            q = torch.randn(B, H, D, device=dev).half()
+            k = torch.randn(B, Hkv, D, device=dev).half()
+            v = torch.randn(B, Hkv, D, device=dev).half()
+            us = timed(lambda: [eng.single_query_attention(q, k, v, kc, vc, None, None, t, D, 1000000.0, 1.0, True)
+                                for kc, vc in zip(kcs, vcs)]) / n
+            row = {"G": G, "kernel": "tensor_core" if G > 8 else "cuda_core", "us": round(us, 3), "kv_bytes": b,
+                   "GBs": round(b / us / 1e3, 1), "hbm_frac": round(b / us / 1e3 / peaks["hbm"], 3), "caches_per_replay": n}
+            if G > 8:
+                flop = 4 * B * H * (t + 1) * D
+                t_hbm, t_tc = b / (peaks["hbm"] * 1e3), flop / (peaks["tc_burst"] * 1e6)   # us
+                row.update({"flop": flop, "TFLOPs": round(flop / us / 1e6, 2), "bound": "hbm" if t_hbm >= t_tc else "tensor",
+                            "hbm_bound_us": round(t_hbm, 3), "tc_bound_us": round(t_tc, 3)})
+            out["attention_%s_b%d_ctx%d" % (name, B, L)] = row
+            del kcs, vcs
+out["peaks"] = dict(peaks)
+try:
+    import subprocess
+    out["device"] = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                   capture_output=True, text=True).stdout.strip()
+except OSError:
+    out["device"] = torch.cuda.get_device_name(0)
 print(json.dumps(out, indent=1))
